@@ -4,6 +4,7 @@ seidel path.  Contract: see the task statement; one JSON line on stdout (rank 0)
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo (CUDA kernels)
   python bench.py --impl reference [--gpus N] [--steps K] ...    # the reference's own CPU path on the host cores
+  python bench.py --dump-outputs DIR ...                         # also write the last timed step's results to DIR
 
 A "step" = one pass of the hot path over one batch of `--batch` synthetic paths per GPU (BASELINE.json configs[1]:
 4096 random 7-DOF spline paths, 200 gridpoints, vel+acc): K0 spline fit -> K1 coefficient records -> K2
@@ -19,6 +20,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the benchmark leaves the tree it runs from untouched (it may be read-only)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -47,7 +49,31 @@ def parse_args():
                     "headline cfg 2 (comma list out of 1,3,4,5; 'none' to skip)")
     ap.add_argument("--cfg3-batch", type=int, default=65536)
     ap.add_argument("--cfg5-batch", type=int, default=1 << 20)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write K, sd, u, status, fail_stage of the last timed step of "
+                    "the headline path as DIR/<name>.npy (float64; rank 0's shard), for comparing two builds")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out, directory):
+    """Writes the arrays the headline path returns as float64 .npy files.  The inputs are seeded, so two builds run with
+    the same arguments can be compared file by file.  If the batch exceeds DUMP_LIMIT_BYTES, a fixed seeded sample of
+    paths is written; path_index.npy always lists the paths (rows) written."""
+    host = {k: v.cpu().numpy().astype(np.float64) for k, v in out.items() if v is not None}
+    B = host["K"].shape[0]
+    per_path = sum(a[0].nbytes for a in host.values()) + 8
+    idx = np.arange(B)
+    if per_path * B > DUMP_LIMIT_BYTES:
+        idx = np.sort(np.random.RandomState(0).choice(B, DUMP_LIMIT_BYTES // per_path, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "path_index.npy"), idx.astype(np.float64))
+    for name, a in host.items():
+        np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a[idx]))
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -523,6 +549,7 @@ def run_b200(args):
     k_events = []  # (k0_start, k1_start, k2_start, k2_end) per timed step
 
     scan_mode = {"fast_lower": False}
+    last_out = {}   # results of the latest timed headline step (for --dump-outputs)
 
     xbound = torch.empty((B, G, 2), dtype=torch.float64, device=dev)
 
@@ -539,6 +566,8 @@ def run_b200(args):
         if e:
             e[3].record()
             k_events.append(e)
+            if args.dump_outputs and len(k_events) == args.steps:   # keep nothing alive between timed steps
+                last_out["out"] = out
         return out
 
     rec_events = []
@@ -669,6 +698,8 @@ def run_b200(args):
         clocks_first = clocks
         ms_dev, ms_e2e, ms_e2e_sync, clocks = measure()
         clocks["remeasured_after"] = clocks_first
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last_out["out"], args.dump_outputs)
 
     # opt-in mode (BatchTOPPRA(exact=False), TB_SCAN_FAST_LOWER): reported beside the headline, never instead of it
     scan_mode["fast_lower"] = True

@@ -7,7 +7,7 @@ import toppra_b200 as ta
 from problems import SHORTCUT_SETS
 from oracle import oracle as orc
 name = "scaled14"
-g = np.load(os.path.join(ROOT, "tests", "golden", "shortcut_rows.npz"))
+g = np.load(os.path.join(ROOT, "tests", "golden", "shortcut_rows_%s.npz" % name))
 gen, args = SHORTCUT_SETS[name]
 rows, xb = gen(*args)
 B, G, _, R = rows.shape

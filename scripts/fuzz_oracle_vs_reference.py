@@ -5,7 +5,10 @@ UNMODIFIED reference build (oracle/_ref) on randomly SHAPED problems — far mor
 and interpolation, active velocity bounds, non-zero boundary velocities (admissible or not), near-degenerate paths.
 Any mismatch is printed with the seed that reproduces it.
 
-usage: python scripts/fuzz_oracle_vs_reference.py [--minutes M] [--seed S]      (needs oracle/_ref, i.e. this container)"""
+usage: python scripts/fuzz_oracle_vs_reference.py [--minutes M] [--seed S]      (needs the reference build, oracle/_ref)
+
+Every result of the reference goes through `theirs()`, so a slice of the campaign can be recorded once
+(tests/golden/make_golden.py fuzz_slice) and replayed without the reference (tests/test_oracle_vs_reference.py)."""
 import argparse
 import os
 import sys
@@ -19,16 +22,141 @@ sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
 warnings.filterwarnings("ignore")
 
 from oracle import oracle as orc  # noqa: E402
-from oracle.ref_loader import load_reference  # noqa: E402
 
-ta = load_reference()
-import toppra.algorithm as algo  # noqa: E402
-import toppra.constraint as constraint  # noqa: E402
-import toppra.interpolator as interp  # noqa: E402
-from toppra.parametrizer import ParametrizeSpline  # noqa: E402
+ta = algo = constraint = interp = ParametrizeSpline = None
+
+
+def load():
+    """Import the reference build (oracle/_ref) for live runs."""
+    global ta, algo, constraint, interp, ParametrizeSpline
+    from oracle.ref_loader import load_reference
+    ta = load_reference()
+    import toppra.algorithm as algo
+    import toppra.constraint as constraint
+    import toppra.interpolator as interp
+    from toppra.parametrizer import ParametrizeSpline
+
+
+REPLAY = None      # {key: array}: the reference's results as recorded into RECORD; None = call the reference
+RECORD = None      # dict that collects the reference's results of a live run (stored with pack())
+_PREFIX = [""]
+
+
+class ReferenceRaised(Exception):
+    """Replay of a reference call that raised."""
+
+
+def begin(seed):
+    """Key the reference's results of the next problem by its seed."""
+    _PREFIX[0] = "%d/" % seed
+
+
+def _encode(key, value, out, digest):
+    if digest and not isinstance(value, (str, tuple, list)) and value is not None and np.size(value) > 1:
+        d = Digest.of(value)
+        out[key + "!shape"], out[key + "!sha256"] = np.array(d.shape, dtype=np.int64), np.array(d.sha)
+    elif value is None:
+        out[key + "!none"] = np.array(True)
+    elif isinstance(value, str):
+        out[key + "!str"] = np.array(value)
+    elif isinstance(value, (tuple, list)):
+        out[key + "!len"] = np.array(len(value))
+        for i, v in enumerate(value):
+            _encode("%s/%d" % (key, i), v, out, digest)
+    else:
+        out[key] = np.asarray(value)
+
+
+def _decode(key, data):
+    if not any(k in data for k in (key, key + "!raise", key + "!none", key + "!str", key + "!len", key + "!sha256")):
+        raise AssertionError("no recorded reference result for " + key)
+    if key + "!raise" in data:
+        raise ReferenceRaised(str(data[key + "!raise"]))
+    if key + "!none" in data:
+        return None
+    if key + "!sha256" in data:
+        return Digest(data[key + "!shape"], data[key + "!sha256"])
+    if key + "!str" in data:
+        return str(data[key + "!str"])
+    if key + "!len" in data:
+        return tuple(_decode("%s/%d" % (key, i), data) for i in range(int(data[key + "!len"])))
+    return data[key]
+
+
+def pack(record):
+    """RECORD as five arrays (keys, kinds, shapes, numbers, strings): one file entry per key would cost more than the data."""
+    keys = sorted(record)
+    kinds, shapes, nums, strs = [], [], [], []
+    for k in keys:
+        v = np.asarray(record[k])
+        if v.dtype.kind == "U":
+            kinds.append(1)
+            strs.append(str(v))
+        else:
+            kinds.append(0)
+            shapes += [v.ndim] + list(v.shape)
+            nums.append(v.astype(np.float64).ravel())
+    return {"keys": np.array(keys), "kinds": np.array(kinds, dtype=np.int8), "shapes": np.array(shapes, dtype=np.int64),
+            "numbers": np.concatenate(nums) if nums else np.zeros(0), "strings": np.array(strs)}
+
+
+def unpack(packed):
+    """The inverse of pack()."""
+    out, shapes, nums, strs = {}, iter(packed["shapes"].tolist()), packed["numbers"], iter(packed["strings"].tolist())
+    pos = 0
+    for k, kind in zip(packed["keys"].tolist(), packed["kinds"].tolist()):
+        if kind == 1:
+            out[k] = np.array(next(strs))
+        else:
+            shape = tuple(next(shapes) for _ in range(next(shapes)))
+            n = int(np.prod(shape))
+            out[k] = nums[pos:pos + n].reshape(shape)
+            pos += n
+    return out
+
+
+def theirs(what, fn, digest=True):
+    """The reference's result `fn()` (arrays, numbers, strings, None or tuples of them): live, recorded, or replayed.
+    digest=True: its arrays are only compared with eq(), so a recording keeps their digests; digest=False for results
+    that are computed with or compared to a tolerance."""
+    key = _PREFIX[0] + what
+    if REPLAY is not None:
+        return _decode(key, REPLAY)
+    try:
+        value = fn()
+    except Exception as e:
+        if RECORD is not None:
+            RECORD[key + "!raise"] = np.array(type(e).__name__)
+        raise
+    if RECORD is not None:
+        _encode(key, value, RECORD, digest)
+    return value
+
+
+class Digest(object):
+    """A recorded reference array that is only ever compared bit for bit (eq): its shape and a SHA-256 of its values with
+    NaNs and signed zeros folded, so that two arrays have the same digest exactly when eq() holds for them."""
+
+    def __init__(self, shape, sha):
+        self.shape, self.sha = tuple(int(n) for n in shape), str(sha)
+
+    @staticmethod
+    def of(a):
+        import hashlib
+        a = np.asarray(a, dtype=float)
+        a = np.where(np.isnan(a), np.nan, a) + 0.0
+        return Digest(a.shape, hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest())
+
+    def __len__(self):
+        return self.shape[0]
+
+    def __eq__(self, other):
+        return isinstance(other, Digest) and (self.shape, self.sha) == (other.shape, other.sha)
 
 
 def eq(a, b):
+    if isinstance(a, Digest) or isinstance(b, Digest):
+        return (a if isinstance(a, Digest) else Digest.of(a)) == (b if isinstance(b, Digest) else Digest.of(b))
     return np.array_equal(np.asarray(a, dtype=float), np.asarray(b, dtype=float), equal_nan=True)
 
 
@@ -36,9 +164,28 @@ from problems import random_shaped_problem as random_problem  # noqa: E402
 
 
 def check_solve(p):
-    path = ta.SplineInterpolator(p["ss"], p["way"], bc_type=p["bc"])
+    def spline():
+        path = ta.SplineInterpolator(p["ss"], p["way"], bc_type=p["bc"])
+        return path.cspl.c if p["way"].shape[0] > 1 else None
+
+    def solve():
+        path = ta.SplineInterpolator(p["ss"], p["way"], bc_type=p["bc"])
+        cons = [constraint.JointVelocityConstraint(p["vlim"]),
+                constraint.JointAccelerationConstraint(p["alim"], discretization_scheme=p["interp"])]
+        inst = algo.TOPPRA(cons, path, gridpoints=p["grid"], solver_wrapper="seidel")
+        sdd, sd, _, K = inst.compute_parameterization(p["sd0"], p["sd1"], return_data=True)
+        code = inst.problem_data.return_code
+        assert algo.ParameterizationReturnCode.__members__[code.name] is code
+        return sdd, sd, K, code.name
+
+    def feasible_sets():
+        path = ta.SplineInterpolator(p["ss"], p["way"], bc_type=p["bc"])
+        cons = [constraint.JointVelocityConstraint(p["vlim"]),
+                constraint.JointAccelerationConstraint(p["alim"], discretization_scheme=p["interp"])]
+        return algo.TOPPRA(cons, path, gridpoints=p["grid"], solver_wrapper="seidel").compute_feasible_sets()
+
     c = orc.cubic_spline_fit(p["ss"], p["way"], p["bc"])
-    ref_c = path.cspl.c if p["way"].shape[0] > 1 else None
+    ref_c = theirs("spline", spline, digest=False)
     if p["bc"] == "not-a-knot" and len(p["ss"]) != 3:
         assert eq(c, ref_c), "spline coefficients"
     else:
@@ -47,19 +194,14 @@ def check_solve(p):
         # with the reference's coefficients so that everything downstream is compared bit for bit
         np.testing.assert_allclose(c, ref_c, rtol=1e-11, atol=1e-12 * max(1.0, np.abs(ref_c).max()))
         c = np.ascontiguousarray(ref_c)
-    cons = [constraint.JointVelocityConstraint(p["vlim"]),
-            constraint.JointAccelerationConstraint(p["alim"], discretization_scheme=p["interp"])]
-    inst = algo.TOPPRA(cons, path, gridpoints=p["grid"], solver_wrapper="seidel")
-    sdd, sd, _, K = inst.compute_parameterization(p["sd0"], p["sd1"], return_data=True)
+    sdd, sd, K, code = theirs("solve", solve)
     o = orc.solve_velacc(c, p["ss"], p["grid"], p["vlim"], p["alim"], bool(p["interp"]), p["sd0"], p["sd1"])
     assert eq(o["K"], K), "K"
-    code = inst.problem_data.return_code
-    assert algo.ParameterizationReturnCode.__members__[code.name] is code
-    want = {"Ok": 0, "ErrUnknown": 1, "ErrShortPath": 2, "FailUncontrollable": 3, "ErrForwardPassFail": 4}[code.name]
-    assert o["status"] == want, ("status", o["status"], code.name)
+    want = {"Ok": 0, "ErrUnknown": 1, "ErrShortPath": 2, "FailUncontrollable": 3, "ErrForwardPassFail": 4}[code]
+    assert o["status"] == want, ("status", o["status"], code)
     if sd is not None:
         assert eq(o["sd"], sd) and eq(o["u"], sdd), "sd / u"
-    X = algo.TOPPRA(cons, path, gridpoints=p["grid"], solver_wrapper="seidel").compute_feasible_sets()
+    X = theirs("feasible_sets", feasible_sets)
     lin = orc.solve_velacc(c, p["ss"], p["grid"], p["vlim"], p["alim"], bool(p["interp"]), 0, 0, want_rows=True)
     w = orc.Wrapper(p["grid"], lin["rows"], lin["xbound"])
     assert eq(w.compute_feasible_sets(), X), "feasible sets"
@@ -69,16 +211,18 @@ def check_solve(p):
 def check_frows(p, rng):
     if p["way"].shape[0] < 2:
         return
-    path = ta.SplineInterpolator(p["ss"], p["way"])
     c = orc.cubic_spline_fit(p["ss"], p["way"])
     import torch
     import cpu_engine
     kw = dict(max_err_threshold=10 ** rng.uniform(-5, -1), max_seg_length=rng.uniform(0.02, 0.6) * p["ss"][-1],
               min_nb_points=int(rng.randint(2, 200)))
-    try:
-        want = np.asarray(interp.propose_gridpoints(path, **kw))
-    except ValueError:
-        want = None
+    def proposed():
+        try:
+            return np.asarray(interp.propose_gridpoints(ta.SplineInterpolator(p["ss"], p["way"]), **kw))
+        except ValueError:
+            return None
+
+    want = theirs("propose_gridpoints", proposed)
     grid, glen, st = cpu_engine.propose_gridpoints(torch.from_numpy(c[None]), torch.from_numpy(p["ss"]), max_points=8192, **kw)
     if int(st[0]) < 0:
         pass                                    # more than max_points gridpoints needed: the cap of this harness, not a result
@@ -94,14 +238,19 @@ def check_frows(p, rng):
             vel[rng.randint(0, G, size=2)] = 0.0
         if rng.rand() < 0.3:
             vel[G // 3:G // 3 + 2] = 1e10
-        try:
-            traj = ParametrizeSpline(path, p["grid"], vel)
-        except Exception:
+        def knots():
+            try:
+                return ParametrizeSpline(ta.SplineInterpolator(p["ss"], p["way"]), p["grid"], vel).ss_waypoints
+            except Exception:
+                return None
+
+        want = theirs("time_stamps", knots)
+        if want is None:
             return
         t, s, nk = cpu_engine.spline_time_stamps(torch.from_numpy(vel[None]), torch.from_numpy(p["grid"]))
         k = int(nk[0])
         count("time stamps")
-        assert k == len(traj.ss_waypoints) and eq(t[0, :k].numpy(), traj.ss_waypoints), "ParametrizeSpline time stamps"
+        assert k == len(want) and eq(t[0, :k].numpy(), want), "ParametrizeSpline time stamps"
 
 
 _MINE = []
@@ -137,21 +286,25 @@ def check_sd_and_reachable(p, rng):
     tb = mine()
     mk = lambda pkg, cons: [cons.JointVelocityConstraint(p["vlim"]),  # noqa: E731
                             cons.JointAccelerationConstraint(p["alim"], discretization_scheme=p["interp"])]
-    theirs = ta.SplineInterpolator(p["ss"], p["way"])
+    ref_path = lambda: ta.SplineInterpolator(p["ss"], p["way"])  # noqa: E731
     ours = tb.SplineInterpolator(p["ss"], p["way"])
-    fast = algo.TOPPRA(mk(algo, constraint), theirs, gridpoints=p["grid"], solver_wrapper="seidel")
-    _, sd_f, _ = fast.compute_parameterization(0, 0)
+    sd_f = theirs("fast_sd", lambda: algo.TOPPRA(mk(algo, constraint), ref_path(), gridpoints=p["grid"],
+                                                 solver_wrapper="seidel").compute_parameterization(0, 0)[1], digest=False)
     if sd_f is not None and np.all(sd_f[1:] + sd_f[:-1] > 0):
         t_fast = np.sum(2 * np.diff(p["grid"]) / (sd_f[1:] + sd_f[:-1]))
         want_t = t_fast * rng.choice([0.5, 1.0, 1.2, 2.0, 7.0, 1e3])
-        a = algo.TOPPRAsd(mk(algo, constraint), theirs, gridpoints=p["grid"], solver_wrapper="seidel")
+
+        def desired_duration():
+            a = algo.TOPPRAsd(mk(algo, constraint), ref_path(), gridpoints=p["grid"], solver_wrapper="seidel")
+            a.set_desired_duration(want_t)
+            return a.compute_parameterization(0, 0, return_data=True) + (a.problem_data.return_code.name,)
+
+        *ra, code_a = theirs("TOPPRAsd", desired_duration)
         b = tb.algorithm.TOPPRAsd(mk(tb.algorithm, tb.constraint), ours, gridpoints=p["grid"], solver_wrapper="seidel")
-        a.set_desired_duration(want_t)
         b.set_desired_duration(want_t)
-        ra = a.compute_parameterization(0, 0, return_data=True)
         rb = b.compute_parameterization(0, 0, return_data=True)
         count("TOPPRAsd")
-        assert a.problem_data.return_code.name == b.problem_data.return_code.name, "TOPPRAsd return code"
+        assert code_a == b.problem_data.return_code.name, "TOPPRAsd return code"
         for x, y, what in zip(ra, rb, ("sdd", "sd", "v", "K")):
             assert (x is None and y is None) or eq(x, y), "TOPPRAsd " + what
     sdmin = 0.0 if rng.rand() < 0.5 else 10 ** rng.uniform(-3, -0.5)
@@ -164,7 +317,8 @@ def check_sd_and_reachable(p, rng):
             sdmin = val
         else:
             sdmax = val
-    La = algo.TOPPRA(mk(algo, constraint), theirs, gridpoints=p["grid"], solver_wrapper="seidel").compute_reachable_sets(sdmin, sdmax)
+    La = theirs("reachable_sets", lambda: algo.TOPPRA(mk(algo, constraint), ref_path(), gridpoints=p["grid"],
+                                                      solver_wrapper="seidel").compute_reachable_sets(sdmin, sdmax))
     Lb = tb.algorithm.TOPPRA(mk(tb.algorithm, tb.constraint), ours, gridpoints=p["grid"],
                              solver_wrapper="seidel").compute_reachable_sets(sdmin, sdmax)
     count("reachable sets")
@@ -176,27 +330,40 @@ def check_parametrizers(p, rng):
     (knot times bit for bit, the clamped re-fit and its evaluations to rounding) on the solved velocity profile."""
     if p["bc"] != "not-a-knot" or len(p["ss"]) == 3 or len(p["grid"]) < 3:
         return
-    from toppra.parametrizer import ParametrizeConstAccel
     tb = mine()
-    theirs, ours = ta.SplineInterpolator(p["ss"], p["way"]), tb.SplineInterpolator(p["ss"], p["way"])
-    cons = [constraint.JointVelocityConstraint(p["vlim"]), constraint.JointAccelerationConstraint(p["alim"], p["interp"])]
-    _, sd, _ = algo.TOPPRA(cons, theirs, gridpoints=p["grid"], solver_wrapper="seidel").compute_parameterization(0, 0)
+    ref_path = lambda: ta.SplineInterpolator(p["ss"], p["way"])  # noqa: E731
+    ours = tb.SplineInterpolator(p["ss"], p["way"])
+
+    def velocities():
+        cons = [constraint.JointVelocityConstraint(p["vlim"]), constraint.JointAccelerationConstraint(p["alim"], p["interp"])]
+        return algo.TOPPRA(cons, ref_path(), gridpoints=p["grid"], solver_wrapper="seidel").compute_parameterization(0, 0)[1]
+
+    def const_accel():
+        from toppra.parametrizer import ParametrizeConstAccel
+        return ParametrizeConstAccel(ref_path(), p["grid"], sd)
+
+    sd = theirs("parametrizer_sd", velocities, digest=False)
     if sd is None or not np.all(sd[1:] + sd[:-1] > 0):
         return
-    a, b = ParametrizeConstAccel(theirs, p["grid"], sd), tb.ParametrizeConstAccel(ours, p["grid"], sd)
+    a_ts, a_us, a_duration = theirs("ConstAccel", lambda: (lambda a: (a._ts, a._us, a.duration))(const_accel()))
+    b = tb.ParametrizeConstAccel(ours, p["grid"], sd)
     count("ParametrizeConstAccel")
-    assert eq(a._ts, b._ts) and eq(a._us, b._us) and a.duration == b.duration, "ConstAccel time grid"
-    ts = np.r_[0.0, np.sort(rng.uniform(0, a.duration, 30)), a.duration]
+    assert eq(a_ts, b._ts) and eq(a_us, b._us) and a_duration == b.duration, "ConstAccel time grid"
+    ts = np.r_[0.0, np.sort(rng.uniform(0, a_duration, 30)), a_duration]
     scale = max(1.0, np.abs(p["way"]).max())
+    wants = theirs("ConstAccel_eval", lambda: (lambda a: [a(ts, order) for order in (0, 1, 2)])(const_accel()),
+                   digest=False)
     for order, tol in ((0, 1e-11), (1, 1e-9), (2, 1e-7)):
-        want = a(ts, order)
+        want = wants[order]
         np.testing.assert_allclose(b(ts, order), want, rtol=tol, atol=tol * max(scale, np.abs(want).max()),
                                    err_msg="ConstAccel order %d" % order)
-    sa, sb = ParametrizeSpline(theirs, p["grid"], sd), tb.ParametrizeSpline(ours, p["grid"], sd)
+    sa_knots, sa_duration = theirs("Spline", lambda: (lambda s: (s.ss_waypoints, s.duration))(
+        ParametrizeSpline(ref_path(), p["grid"], sd)))
+    sb = tb.ParametrizeSpline(ours, p["grid"], sd)
     count("ParametrizeSpline")
-    assert eq(sa.ss_waypoints, sb.ss_waypoints) and sa.duration == sb.duration, "ParametrizeSpline knots"
-    ts = np.linspace(0, sa.duration, 25)
-    want = sa(ts)
+    assert eq(sa_knots, sb.ss_waypoints) and sa_duration == sb.duration, "ParametrizeSpline knots"
+    ts = np.linspace(0, sa_duration, 25)
+    want = theirs("Spline_eval", lambda: ParametrizeSpline(ref_path(), p["grid"], sd)(ts), digest=False)
     np.testing.assert_allclose(sb(ts), want, rtol=1e-9, atol=1e-9 * max(scale, np.abs(want).max()), err_msg="ParametrizeSpline q")
 
 
@@ -230,16 +397,17 @@ def check_ubound(p, rng):
     width = 10 ** rng.uniform(-1.5, 1.0) * max(1e-3, np.abs(p["alim"]).max())
     ub = np.stack((-width * (0.5 + rng.rand(G)), width * (0.5 + rng.rand(G))), axis=1)
     xb = np.stack((np.zeros(G), 10 ** rng.uniform(-2, 3) * (0.5 + rng.rand(G))), axis=1)
-    out = []
-    for pkg, cons, path in ((algo, constraint, ta.SplineInterpolator(p["ss"], p["way"])),
-                            (tb.algorithm, tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))):
+    def run(pkg, cons, path):
         mk = lambda: [cons.JointVelocityConstraint(p["vlim"]),  # noqa: E731
                       _ub_class(cons)(cons.JointAccelerationConstraint(p["alim"], p["interp"]), ub, xb)]
         inst = pkg.TOPPRA(mk(), path, gridpoints=p["grid"], solver_wrapper="seidel")
         res = inst.compute_parameterization(0, 0, return_data=True)
         X = pkg.TOPPRA(mk(), path, gridpoints=p["grid"], solver_wrapper="seidel").compute_feasible_sets()
         L = pkg.TOPPRA(mk(), path, gridpoints=p["grid"], solver_wrapper="seidel").compute_reachable_sets(0.0, 0.25)
-        out.append((res[0], res[1], res[3], X, L))
+        return (res[0], res[1], res[3], X, L)
+
+    out = [theirs("ubound", lambda: run(algo, constraint, ta.SplineInterpolator(p["ss"], p["way"]))),
+           run(tb.algorithm, tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))]
     count("ubound")
     for x, y, what in zip(out[0], out[1], ("sdd", "sd", "K", "feasible sets", "reachable sets")):
         assert (x is None and y is None) or (x is not None and y is not None and eq(x, y)), "ubound " + what
@@ -254,9 +422,7 @@ def check_other_constraints(p, rng):
     tb = mine()
     k0, k1 = 0.05 + rng.rand(), rng.rand() / p["ss"][-1]
     vlim, span = p["vlim"], p["ss"][-1]
-    out = []
-    for pkg, cons, path in ((algo, constraint, ta.SplineInterpolator(p["ss"], p["way"])),
-                            (tb.algorithm, tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))):
+    def run(pkg, cons, path):
         var = cons.JointVelocityConstraintVarying(lambda s: vlim * (k0 + k1 * s))
         inst = pkg.TOPPRA([var, cons.JointAccelerationConstraint(p["alim"], p["interp"])], path, gridpoints=p["grid"],
                           solver_wrapper="seidel")
@@ -269,7 +435,10 @@ def check_other_constraints(p, rng):
                               solver_wrapper="seidel")
             res = inst.compute_parameterization(0, 0, return_data=True)
             item += [res[0], res[1], res[3]]
-        out.append(item)
+        return item
+
+    out = [theirs("other_constraints", lambda: run(algo, constraint, ta.SplineInterpolator(p["ss"], p["way"]))),
+           run(tb.algorithm, tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))]
     count("varying velocity limits" + (" + JointTorqueConstraint" if len(out[0]) > 4 else ""))
     names = ("varying: sdd", "varying: sd", "varying: K", "varying: xbound", "joint torque: sdd", "joint torque: sd",
              "joint torque: K")
@@ -297,13 +466,17 @@ def check_batch(p, rng):
     ragged = ragged_inst.compute_parameterization(sd0, 0.0).to_host()
     glen = ragged_inst.glen.cpu().numpy()
     count("batch (common + ragged grids)")
-    for b in range(B):
+    def solve(b, grid):
         path = ta.SplineInterpolator(p["ss"], way[b])
         cons = [constraint.JointVelocityConstraint(vlim[b]), constraint.JointAccelerationConstraint(alim[b], p["interp"])]
+        inst = algo.TOPPRA(cons, path, gridpoints=grid, solver_wrapper="seidel")
+        sdd, sd, _, K = inst.compute_parameterization(float(sd0[b]), 0.0, return_data=True)
+        return sdd, sd, K, len(inst.gridpoints)
+
+    for b in range(B):
         for grid, got, tag in ((p["grid"], common, "common grid"), (None, ragged, "proposed grid")):
-            inst = algo.TOPPRA(cons, path, gridpoints=grid, solver_wrapper="seidel")
-            sdd, sd, _, K = inst.compute_parameterization(float(sd0[b]), 0.0, return_data=True)
-            G = len(inst.gridpoints)
+            sdd, sd, K, G = theirs("batch/%d/%s" % (b, tag), lambda: solve(b, grid))
+            G = int(G)
             if grid is None:
                 assert glen[b] == G, "batch: proposed grid length"
             assert eq(got["K"][b, :G], K), "batch K (%s)" % tag
@@ -320,10 +493,12 @@ def check_robust_params(p, rng):
         return
     tb = mine()
     ell = list(10 ** rng.uniform(-4, 0, 3))
-    out = []
-    for cons, path in ((constraint, ta.SplineInterpolator(p["ss"], p["way"])), (tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))):
+    def run(cons, path):
         base = cons.JointAccelerationConstraint(p["alim"], p["interp"])
-        out.append(cons.RobustLinearConstraint(base, ell, p["interp"]).compute_constraint_params(path, p["grid"]))
+        return cons.RobustLinearConstraint(base, ell, p["interp"]).compute_constraint_params(path, p["grid"])
+
+    out = [theirs("robust_params", lambda: run(constraint, ta.SplineInterpolator(p["ss"], p["way"]))),
+           run(tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))]
     count("robust parameters")
     assert len(out[0]) == len(out[1]), "robust tuple length"
     for x, y, what in zip(out[0], out[1], ("a", "b", "c", "P", "ubound", "xbound")):
@@ -341,19 +516,34 @@ def check_torque(p, rng):
     taulim = np.stack((-(20 + 30 * rng.rand(dof)), 20 + 30 * rng.rand(dof)), axis=1)
     fric = np.zeros(dof) if rng.rand() < 0.5 else 0.5 * rng.rand(dof)
     scheme = int(rng.rand() < 0.6)
-    out = []
-    for pkg, cons, path in ((algo, constraint, ta.SplineInterpolator(p["ss"], p["way"])),
-                            (tb.algorithm, tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))):
+    def run(pkg, cons, path):
         torque = cons.SecondOrderConstraint.joint_torque_constraint(inv_dyn_numpy, taulim, fric,
                                                                     discretization_scheme=scheme)
         inst = pkg.TOPPRA([cons.JointVelocityConstraint(p["vlim"]), cons.JointAccelerationConstraint(p["alim"]), torque],
                           path, gridpoints=p["grid"], solver_wrapper="seidel")
-        out.append(inst.compute_parameterization(p["sd0"], p["sd1"], return_data=True) +
-                   (inst.problem_data.return_code.name,))
+        return inst.compute_parameterization(p["sd0"], p["sd1"], return_data=True) + (inst.problem_data.return_code.name,)
+
+    out = [theirs("torque", lambda: run(algo, constraint, ta.SplineInterpolator(p["ss"], p["way"]))),
+           run(tb.algorithm, tb.constraint, tb.SplineInterpolator(p["ss"], p["way"]))]
     count("torque (%s)" % out[0][-1])
     for x, y, what in zip(out[0], out[1], ("sdd", "sd", "v", "K", "return code")):
         same = (x == y) if isinstance(x, str) else ((x is None and y is None) or (x is not None and y is not None and eq(x, y)))
         assert same, "torque " + what
+
+
+def check_all(p, rng):
+    """Every check on one problem; AssertionError on a mismatch, any other exception where the reference rejected the input.
+    Returns the reference's status code."""
+    st = check_solve(p)
+    check_frows(p, rng)
+    check_sd_and_reachable(p, rng)
+    check_torque(p, rng)
+    check_parametrizers(p, rng)
+    check_ubound(p, rng)
+    check_other_constraints(p, rng)
+    check_batch(p, rng)
+    check_robust_params(p, rng)
+    return st
 
 
 def main():
@@ -361,22 +551,15 @@ def main():
     ap.add_argument("--minutes", type=float, default=5.0)
     ap.add_argument("--seed", type=int, default=0)
     args = ap.parse_args()
+    load()
     t_end = time.time() + 60 * args.minutes
     seed, bad, hist = args.seed, [], {}
     while time.time() < t_end:
         rng = np.random.RandomState(seed)
         p = random_problem(rng)
         try:
-            st = check_solve(p)
+            st = check_all(p, rng)
             hist[st] = hist.get(st, 0) + 1
-            check_frows(p, rng)
-            check_sd_and_reachable(p, rng)
-            check_torque(p, rng)
-            check_parametrizers(p, rng)
-            check_ubound(p, rng)
-            check_other_constraints(p, rng)
-            check_batch(p, rng)
-            check_robust_params(p, rng)
         except AssertionError as e:
             bad.append((seed, str(e)[:200]))
             print("MISMATCH seed %d: %s  (dof %d, n %d, G %d, bc %s, interp %d, sd %.3g -> %.3g)"

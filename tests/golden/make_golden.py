@@ -364,7 +364,6 @@ def shortcut_rows_case():
                     self.xb.copy())
 
     codes = list(algo.ParameterizationReturnCode)
-    data = {}
     for name, (gen, args) in SHORTCUT_SETS.items():
         rows, xb = gen(*args)
         B, G = rows.shape[:2]
@@ -378,9 +377,10 @@ def shortcut_rows_case():
             status[i] = codes.index(inst.problem_data.return_code)
             if s_ is not None:
                 sd[i], sdd[i] = s_, u_
-        data.update({name + "_K": K, name + "_sd": sd, name + "_sdd": sdd, name + "_status": status})
+        data = {name + "_K": K, name + "_sd": sd, name + "_sdd": sdd, name + "_status": status}
         print("shortcut rows", name, "status histogram", np.bincount(status, minlength=5))
-    np.savez_compressed(os.path.join(HERE, "shortcut_rows.npz"), **data)
+        # one file per set keeps every fixture under 1 MB
+        np.savez_compressed(os.path.join(HERE, "shortcut_rows_%s.npz" % name), **data)
 
 
 def joint_torque_case():
@@ -588,9 +588,213 @@ def frows_batch_case():
           "| ubound status", ub_status)
 
 
+def oracle_vs_reference_case():
+    """The reference's outputs on the random problems of tests/test_oracle_vs_reference.py (same seeds, same inputs),
+    and the reference's public API (classes, members, argument names) for the introspection test there."""
+    import json
+    import inspect
+    import toppra.interpolator as interp
+    import toppra.parametrizer
+    import toppra.simplepath
+    import toppra.solverwrapper
+    from toppra.parametrizer import ParametrizeSpline
+    data = {}
+    ss = np.linspace(0, 1, 5)
+    # test_random_paths_bit_exact
+    for vel_active in (0, 1):
+        for seed in range(5000, 5040):
+            key = "paths%d_%d_" % (vel_active, seed)
+            grid = np.linspace(0, 1, 60 + (seed % 5) * 35)
+            way, vlim, alim = make_path(seed, vel_active=bool(vel_active))
+            path = ta.SplineInterpolator(ss, way)
+            inst = algo.TOPPRA([constraint.JointVelocityConstraint(vlim), constraint.JointAccelerationConstraint(alim)],
+                               path, gridpoints=grid, solver_wrapper="seidel")
+            sdd, sd, _, K = inst.compute_parameterization(0.0 if seed % 3 else 0.02, 0.0, return_data=True)
+            data.update({key + "c": path.cspl.c, key + "K": K})
+            if sd is not None:
+                data.update({key + "sd": sd, key + "sdd": sdd})
+    # test_lp_shims_random
+    rng = np.random.RandomState(0)
+    lp = {"ok": [], "val": [], "var": [], "act": []}
+    for trial in range(300):
+        n = rng.randint(1, 40)
+        v = rng.randn(3)
+        a, b = rng.randn(2, n)
+        c = -rng.rand(n) if trial % 2 else rng.randn(n) * 0.3 - 0.5
+        act = rng.randint(-4, n + 2, size=2)
+        r, val, var, act_out = seidel.solve_lp2d(v, a, b, c, np.r_[-1.0, -2.0], np.r_[1.5, 0.7], act.astype(np.int64))
+        lp["ok"].append(bool(r))
+        lp["val"].append(val if r else np.nan)
+        lp["var"].append(np.asarray(var, dtype=float) if r else np.full(2, np.nan))
+        lp["act"].append(np.asarray(act_out, dtype=np.int64) if r else np.full(2, -99, dtype=np.int64))
+    data.update({"lp_" + k: np.array(v) for k, v in lp.items()})
+    # test_ubound_random_vs_reference
+    rng = np.random.RandomState(17)
+
+    class UB(constraint.LinearConstraint):
+        def __init__(self, acc, ub, xb):
+            super(UB, self).__init__()
+            self.acc, self.ub, self.xb = acc, ub, xb
+            self.discretization_type = acc.discretization_type
+            self.identical = True
+
+        def get_dof(self):
+            return self.acc.get_dof()
+
+        def compute_constraint_params(self, path, gridpoints, *a):
+            pa, pb, pc, F, g, _, _ = self.acc.compute_constraint_params(path, gridpoints)
+            return pa, pb, pc, F, g, self.ub, self.xb
+
+    for seed in range(6000, 6012):
+        key = "ubound_%d_" % seed
+        G = 40 + (seed % 4) * 25
+        grid = np.linspace(0, 1, G)
+        way, vlim, alim = make_path(seed)
+        width = 0.05 + 1.5 * rng.rand()
+        ub = np.stack((-width * (0.5 + rng.rand(G)), width * (0.5 + rng.rand(G))), axis=1)
+        xb = np.stack((np.zeros(G), 20.0 + 80 * rng.rand(G)), axis=1)
+        path = ta.SplineInterpolator(ss, way)
+        mk = lambda: [constraint.JointVelocityConstraint(vlim),  # noqa: E731
+                      UB(constraint.JointAccelerationConstraint(alim), ub, xb)]
+        sdd, sd, _, K = algo.TOPPRA(mk(), path, gridpoints=grid, solver_wrapper="seidel").compute_parameterization(
+            0, 0, return_data=True)
+        data[key + "K"] = K
+        if sd is not None:
+            data.update({key + "sd": sd, key + "sdd": sdd})
+        data[key + "X"] = algo.TOPPRA(mk(), path, gridpoints=grid, solver_wrapper="seidel").compute_feasible_sets()
+        data[key + "L"] = algo.TOPPRA(mk(), path, gridpoints=grid, solver_wrapper="seidel").compute_reachable_sets(0.0, 0.2)
+    # test_propose_gridpoints_and_spline_time_stamps_random_vs_reference
+    rng = np.random.RandomState(23)
+    for seed in range(7000, 7008):
+        key = "grid_%d_" % seed
+        way, _, _ = make_path(seed, dof=3 + seed % 4)
+        path = ta.SplineInterpolator(ss, way)
+        kw = dict(max_err_threshold=10 ** rng.uniform(-4, -1.5), max_seg_length=rng.uniform(0.04, 0.4),
+                  min_nb_points=int(rng.randint(5, 150)))
+        data[key + "proposed"] = np.asarray(interp.propose_gridpoints(path, **kw))
+        G = 80
+        vel = np.abs(rng.randn(G)) + 0.05
+        vel[rng.randint(1, G - 1, size=3)] = 0.0
+        vel[10:12] = 1e9
+        data[key + "time_stamps"] = np.asarray(ParametrizeSpline(path, np.linspace(0, 1, G), vel).ss_waypoints)
+    # test_toppra_sd_random_vs_reference
+    rng = np.random.RandomState(31)
+    for seed in range(8000, 8010):
+        key = "sd_%d_" % seed
+        grid = np.linspace(0, 1, 50 + (seed % 3) * 30)
+        way, vlim, alim = make_path(seed, vel_active=(seed % 4 == 0))
+        mk = lambda: [constraint.JointVelocityConstraint(vlim), constraint.JointAccelerationConstraint(alim)]  # noqa: E731
+        inst = algo.TOPPRAsd(mk(), ta.SplineInterpolator(ss, way), gridpoints=grid, solver_wrapper="seidel")
+        fast = algo.TOPPRA(mk(), ta.SplineInterpolator(ss, way), gridpoints=grid, solver_wrapper="seidel")
+        _, sd_f, _ = fast.compute_parameterization(0, 0)
+        want_t = np.sum(2 * np.diff(grid) / (sd_f[1:] + sd_f[:-1])) * rng.choice([0.6, 1.3, 2.2, 5.0])
+        inst.set_desired_duration(want_t)
+        sdd, sd, _, K = inst.compute_parameterization(0, 0, return_data=True)
+        data.update({key + "duration": np.float64(want_t), key + "K": K, key + "sd": sd, key + "sdd": sdd})
+    # test_univariate_spline_interpolator_vs_reference
+    for seed in range(4):
+        key = "univariate_%d_" % seed
+        rng = np.random.RandomState(900 + seed)
+        n = 25 + 10 * seed
+        s_w = np.sort(np.r_[0.0, rng.uniform(0.05, 2.95, n - 2), 3.0])
+        way = np.stack([np.sin(s_w), np.cos(1.7 * s_w), 0.2 * s_w ** 2 - s_w, np.sin(0.5 * s_w) * s_w], axis=1)
+        way += 0.03 * rng.randn(n, 4)
+        path = ta.UnivariateSplineInterpolator(s_w, way)
+        s = np.linspace(0, 3.0, 301)
+        for order in (0, 1, 2):
+            data[key + "eval%d" % order] = path(s, order)
+        data[key + "dof"] = np.int64(path.dof)
+        data[key + "path_interval"] = np.asarray(path.path_interval, dtype=float)
+        vlim, alim = np.array([[-2.0, 2.0]] * 4), np.array([[-6.0, 5.0]] * 4)
+        inst = algo.TOPPRA([constraint.JointVelocityConstraint(vlim), constraint.JointAccelerationConstraint(alim)], path,
+                           gridpoints=np.linspace(0, 3.0, 151), solver_wrapper="seidel")
+        sdd, sd, _, K = inst.compute_parameterization(0, 0, return_data=True)
+        data.update({key + "K": K, key + "sd": sd, key + "sdd": sdd})
+    # test_public_classes_have_the_reference_methods_and_arguments: {module: {name: {member: [argument names] or None}}}
+    def params(f):
+        try:
+            return [p for p in inspect.signature(f).parameters if p not in ("args", "kwargs")]
+        except (TypeError, ValueError):
+            return None
+
+    api = {}
+    for mod in (ta, algo, constraint, toppra.parametrizer, interp, toppra.simplepath, toppra.solverwrapper):
+        entries = api.setdefault(mod.__name__, {})
+        for name in dir(mod):
+            obj = getattr(mod, name)
+            if name.startswith("_") or not (getattr(obj, "__module__", None) or "").startswith("toppra"):
+                continue
+            if inspect.isclass(obj):
+                members = {}
+                for member in ["__init__"] + [m for m in dir(obj) if not m.startswith("_")]:
+                    fr = getattr(obj, member)
+                    members[member] = params(fr) if callable(fr) and not isinstance(fr, type) else None
+                entries[name] = {"kind": "class", "members": members}
+            elif inspect.isfunction(obj):
+                entries[name] = {"kind": "function", "params": params(obj)}
+    data["public_api_json"] = np.array(json.dumps(api, sort_keys=True))
+    np.savez_compressed(os.path.join(HERE, "oracle_vs_reference.npz"), **data)
+    print("oracle_vs_reference:", len(data), "arrays")
+
+
+def fuzz_slice_case():
+    """The reference's results on the randomly shaped problems of test_randomly_shaped_problems_vs_reference, recorded
+    through the campaign's own checks (scripts/fuzz_oracle_vs_reference.py, `theirs`) while they run live."""
+    import importlib.util
+    from test_oracle_vs_reference import FUZZ_SLICE_SEEDS
+    spec = importlib.util.spec_from_file_location("fuzz_oracle_vs_reference",
+                                                  os.path.join(ROOT, "scripts", "fuzz_oracle_vs_reference.py"))
+    fuzz = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(fuzz)
+    fuzz.load()
+    fuzz.RECORD = {}
+    try:
+        for seed in FUZZ_SLICE_SEEDS:
+            rng = np.random.RandomState(seed)
+            p = fuzz.random_problem(rng)
+            fuzz.begin(seed)
+            try:
+                fuzz.check_all(p, rng)
+            except AssertionError as e:
+                raise AssertionError("seed %d: %s" % (seed, e))
+            except Exception:
+                pass
+    finally:
+        fuzz.release()
+    np.savez_compressed(os.path.join(HERE, "fuzz_slice.npz"), **fuzz.pack(fuzz.RECORD))
+    print("fuzz slice:", len(fuzz.RECORD), "arrays; checks", fuzz.COUNTS)
+
+
+PLUGIN_SINGLE_CASES = [(1000, 200, False, 0.0, 0.0, 1), (1003, 100, True, 0.0, 0.0, 1), (1005, 150, False, 0.1, 0.1, 1),
+                       (1007, 64, False, 0.0, 0.0, 0), (1002, 100, False, 30.0, 0.0, 1)]
+
+
+def plugin_batch_case():
+    """The reference solved path by path on the batch of tests/test_reference_plugin.py (make_batch(24, 1000), 120
+    gridpoints, vel + acc)."""
+    from problems import make_batch
+    ss, way, vlim, alim = make_batch(24, 1000)
+    grid = np.linspace(0, 1, 120)
+    outs = [solve_ref(ss, way[b], vlim[b], alim[b], grid)[0] for b in range(way.shape[0])]
+    data = {k: np.stack([o[k] for o in outs]) for k in ("K", "sd", "sdd", "status")}
+    # single paths with boundary velocities, the collocation scheme and an inadmissible start (status 3)
+    for seed, G, vel_active, s0, s1, scheme in PLUGIN_SINGLE_CASES:
+        way1, vlim1, alim1 = make_path(seed, vel_active=vel_active)
+        o, _ = solve_ref(ss, way1, vlim1, alim1, np.linspace(0, 1, G), s0, s1, scheme)
+        data.update({"single%d_%s" % (seed, k): o[k] for k in ("K", "sd", "sdd", "status")})
+    np.savez_compressed(os.path.join(HERE, "plugin_batch.npz"), **data)
+    print("plugin batch: statuses", data["status"])
+
+
 if __name__ == "__main__":
     if len(sys.argv) > 1 and sys.argv[1] == "shortcut_rows":
         shortcut_rows_case()
+    elif len(sys.argv) > 1 and sys.argv[1] == "oracle_vs_reference":
+        oracle_vs_reference_case()
+    elif len(sys.argv) > 1 and sys.argv[1] == "fuzz_slice":
+        fuzz_slice_case()
+    elif len(sys.argv) > 1 and sys.argv[1] == "plugin_batch":
+        plugin_batch_case()
     elif len(sys.argv) > 1 and sys.argv[1] == "torque_g500":
         torque_g500_case()
     elif len(sys.argv) > 1 and sys.argv[1] == "joint_torque":

@@ -113,7 +113,7 @@ def badly_scaled_rows_batch(R, G, B, seed):
     return rows, xb
 
 
-SHORTCUT_SETS = {  # name -> (generator, args): the problems of tests/golden/shortcut_rows.npz
+SHORTCUT_SETS = {  # name -> (generator, args): the problems of tests/golden/shortcut_rows_<name>.npz
     "deg6": (degenerate_rows_batch, (6, 24, 1500, 105)),
     "deg20": (degenerate_rows_batch, (20, 16, 1500, 119)),
     "scaled14": (badly_scaled_rows_batch, (14, 20, 1200, 6)),

@@ -258,13 +258,13 @@ def test_seidel_shortcuts_on_stress_rows_vs_reference_golden(ta, golden, name):
     fall back to the ordinary walk whenever a decision is close to the TINY threshold.  Raw rows with near-duplicate,
     scaled, parallel and slightly rotated copies (perturbations 1e-14 .. 1e-6) and badly scaled rows (coefficients down
     to 1e-8, optima up to the 1e10 sentinel): 4200 problems, one and two rows per lane, bit for bit against the
-    REFERENCE's own seidelWrapper results (tests/golden/shortcut_rows.npz, generated by make_golden.py shortcut_rows
+    REFERENCE's own seidelWrapper results (tests/golden/shortcut_rows_<set>.npz, generated by make_golden.py shortcut_rows
     from the unmodified reference).  The kernel's per-path re-solve counters must also equal those of the scalar
     shortcut model (oracle/shortcut_model.c), which ties the model campaigns to the kernel's decisions."""
     import torch
     from oracle import oracle as orc
     from problems import SHORTCUT_SETS
-    g = golden("shortcut_rows")
+    g = golden("shortcut_rows_" + name)
     gen, args = SHORTCUT_SETS[name]
     rows, xb = gen(*args)
     B, G, _, R = rows.shape

@@ -272,7 +272,7 @@ def test_shortcut_stress_rows_vs_reference_golden(golden, name):
     The golden holds the REFERENCE's own seidelWrapper results on them (tests/golden/make_golden.py shortcut_rows);
     the restatement must reproduce them bit for bit, so the GPU-vs-oracle tests on these inputs are pinned too."""
     from problems import SHORTCUT_SETS
-    g = golden("shortcut_rows")
+    g = golden("shortcut_rows_" + name)
     gen, args = SHORTCUT_SETS[name]
     rows, xb = gen(*args)
     B, G = rows.shape[:2]

@@ -1,92 +1,56 @@
-"""GPU (-m gpu): the drop-in claim of INTEGRATION.md section 2, executed.  The UNMODIFIED reference (oracle/_ref, built
-from /root/reference by oracle/build_ref.sh and shipped to the GPU box) gets the solver-wrapper name "b200" from
-examples/reference_plugin/b200_solverwrapper.py (pure ctypes over the C-ABI, no torch, none of this repo's Python
-package) and its OWN TOPPRA class must return identical arrays with solver_wrapper="b200" and "seidel" — controllable
-sets, velocities, accelerations, return code and the re-splined trajectory."""
+"""GPU (-m gpu): the batched entry of examples/reference_plugin/b200_solverwrapper.py (pure ctypes over the C-ABI, no
+torch, none of this repo's Python package), the routine that gives the reference the solver-wrapper name "b200", must
+return what the UNMODIFIED reference computes path by path with its own TOPPRA(..., solver_wrapper="seidel").  The
+reference's results are stored in tests/golden/plugin_batch.npz (tests/golden/make_golden.py plugin_batch, whose
+PLUGIN_SINGLE_CASES are the parameters below)."""
 import importlib.util
 import os
 
 import numpy as np
 import pytest
 
-from problems import make_path
-
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope="module")
-def ref():
-    from oracle.ref_loader import load_reference, reference_available
-    if not reference_available():
-        pytest.skip("oracle/_ref (the built reference) is not present")
-    ta = load_reference()
+def plugin():
     spec = importlib.util.spec_from_file_location(
         "b200_solverwrapper", os.path.join(ROOT, "examples", "reference_plugin", "b200_solverwrapper.py"))
-    plugin = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(plugin)
-    plugin.install(ta)
-    return ta, plugin
+    module = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(module)
+    return module
 
 
 @pytest.mark.parametrize("seed,G,vel_active,s0,s1,scheme", [(1000, 200, False, 0.0, 0.0, 1), (1003, 100, True, 0.0, 0.0, 1),
                                                            (1005, 150, False, 0.1, 0.1, 1), (1007, 64, False, 0.0, 0.0, 0),
                                                            (1002, 100, False, 30.0, 0.0, 1)])
-def test_reference_toppra_with_b200_wrapper_equals_seidel(ref, seed, G, vel_active, s0, s1, scheme):
-    ta, _ = ref
-    import toppra.algorithm as algo
-    import toppra.constraint as constraint
+def test_plugin_single_paths_equal_reference(plugin, golden, seed, G, vel_active, s0, s1, scheme):
+    """One path per call, with boundary velocities, the collocation scheme and an inadmissible start: controllable sets,
+    velocities, accelerations and return code of the reference's TOPPRA(..., solver_wrapper="seidel")."""
+    from problems import make_path
     way, vlim, alim = make_path(seed, vel_active=vel_active)
-    ss = np.linspace(0, 1, 5)
-    grid = np.linspace(0, 1, G)
-    out = {}
-    for name in ("seidel", "b200"):
-        path = ta.SplineInterpolator(ss, way)
-        cons = [constraint.JointVelocityConstraint(vlim), constraint.JointAccelerationConstraint(alim, discretization_scheme=scheme)]
-        inst = algo.TOPPRA(cons, path, gridpoints=grid, solver_wrapper=name)
-        sdd, sd, v, K = inst.compute_parameterization(s0, s1, return_data=True)
-        out[name] = (sdd, sd, K, inst.problem_data.return_code)
-    a, b = out["seidel"], out["b200"]
-    assert a[3] == b[3]
-    assert np.array_equal(a[2], b[2], equal_nan=True)
-    if a[1] is None:
-        assert b[1] is None and b[0] is None and s0 == 30.0   # inadmissible start: FailUncontrollable on both
+    ref = golden("plugin_batch")
+    u, sd, K, status = plugin.solve_velacc(np.linspace(0, 1, 5), way[None], np.linspace(0, 1, G), vlim, alim, sd_start=s0,
+                                           sd_end=s1, interpolation=bool(scheme))
+    key = "single%d_" % seed
+    assert status[0] == ref[key + "status"]
+    assert np.array_equal(K[0], ref[key + "K"], equal_nan=True)
+    if status[0] != 0:
+        assert status[0] == 3 and s0 == 30.0   # inadmissible start: FailUncontrollable on both
     else:
-        assert np.array_equal(a[1], b[1]) and np.array_equal(a[0], b[0])
+        assert np.array_equal(sd[0], ref[key + "sd"]) and np.array_equal(u[0], ref[key + "sdd"])
 
 
-def test_reference_compute_trajectory_through_b200(ref):
-    """compute_trajectory (algorithm.py:163-194): the reference's own ParametrizeSpline runs on the arrays of the GPU call."""
-    ta, _ = ref
-    import toppra.algorithm as algo
-    import toppra.constraint as constraint
-    np.random.seed(9)   # examples/plot_kinematics.py:22-33
-    way = np.random.randn(5, 7)
-    vl, al = 10 + np.random.rand(7) * 20, 10 + np.random.rand(7) * 2
-    vlim, alim = np.vstack((-vl, vl)).T, np.vstack((-al, al)).T
-    traj = {}
-    for name in ("seidel", "b200"):
-        inst = algo.TOPPRA([constraint.JointVelocityConstraint(vlim), constraint.JointAccelerationConstraint(alim)],
-                           ta.SplineInterpolator(np.linspace(0, 1, 5), way), solver_wrapper=name)   # automatic gridpoints
-        traj[name] = inst.compute_trajectory(0, 0)
-    ts = np.linspace(0, traj["seidel"].duration, 50)
-    assert traj["b200"].duration == traj["seidel"].duration
-    for order in (0, 1, 2):
-        assert np.array_equal(traj["b200"](ts, order), traj["seidel"](ts, order))
-
-
-def test_plugin_batched_entry_equals_reference(ref):
+def test_plugin_batched_entry_equals_reference(plugin, golden):
     """solve_velacc(B paths) == the reference solved path by path."""
-    ta, plugin = ref
-    import toppra.algorithm as algo
-    import toppra.constraint as constraint
     from problems import make_batch
     B, G = 24, 120
     ss, way, vlim, alim = make_batch(B, 1000)
     grid = np.linspace(0, 1, G)
+    ref = golden("plugin_batch")
     u, sd, K, status = plugin.solve_velacc(ss, way, grid, vlim, alim)
     for b in range(B):
-        inst = algo.TOPPRA([constraint.JointVelocityConstraint(vlim[b]), constraint.JointAccelerationConstraint(alim[b])],
-                           ta.SplineInterpolator(ss, way[b]), gridpoints=grid, solver_wrapper="seidel")
-        sdd_r, sd_r, _, K_r = inst.compute_parameterization(0, 0, return_data=True)
-        assert status[b] == 0 and np.array_equal(K[b], K_r) and np.array_equal(sd[b], sd_r) and np.array_equal(u[b], sdd_r)
+        assert ref["status"][b] == 0
+        assert status[b] == 0 and np.array_equal(K[b], ref["K"][b]) and np.array_equal(sd[b], ref["sd"][b])
+        assert np.array_equal(u[b], ref["sdd"][b])
