@@ -381,10 +381,10 @@ second_order_rows_tiled_kernel(const double *__restrict__ ppoly, const double *_
   }
   for (int t = tid; t < nev; t += SO_THREADS) s_g[t] = gp[gi0 + t];
   // e -> (gridpoint t, joint k) without a division: t = floor(e / dof) by a multiply-high with ceil(2^32 / dof) (exact
-  // for e < 2^16)
-  const unsigned inv_dof = (unsigned)((0x100000000ULL + (unsigned)dof - 1u) / (unsigned)dof);
+  // for e < 2^16).  For dof = 1 that multiplier is 2^32, which does not fit 32 bits: t = e there.
+  const unsigned inv_dof = dof > 1 ? (unsigned)((0x100000000ULL + (unsigned)dof - 1u) / (unsigned)dof) : 0u;
   for (int e = tid; e < nev * dof; e += SO_THREADS) {
-    const int t = (int)__umulhi((unsigned)e, inv_dof), k = e - t * dof;
+    const int t = dof > 1 ? (int)__umulhi((unsigned)e, inv_dof) : e, k = e - t * dof;
     const double s = gp[gi0 + t];
     const int seg = find_interval(x, nseg, s);
     const double q = seg < 0 ? nan_d : ppoly_eval1(cpp, nseg, dof, seg, k, s - x[seg], 0);
@@ -397,7 +397,7 @@ second_order_rows_tiled_kernel(const double *__restrict__ ppoly, const double *_
   }
   __syncthreads();
   for (int e = tid; e < nev * dof; e += SO_THREADS) {
-    const int t = (int)__umulhi((unsigned)e, inv_dof), k = e - t * dof;
+    const int t = dof > 1 ? (int)__umulhi((unsigned)e, inv_dof) : e, k = e - t * dof;
     const double *qd = s_qd + t * dof, *qdd = s_qdd + t * dof, *sq = s_sq + t * dof, *cq = s_cq + t * dof;
     double av, bv, cv;
     if (MODEL == TB_INVDYN_COUPLED_COSINE) {
